@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- attention-forward TFLOP/s on B200 (the one hot path), per the driver contract.
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -375,6 +375,9 @@ def run_ours(args):
         e1.record()
         barrier()
     launches = tfa.launch_count() - n0
+    result = fused.buf if fused is not None else (o_full if world > 1 else out)      # (B,H,S,D) at N>1, local at N=1
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"out": result.view(-1, D), "lse": lse.view(-1)})
     t_total = e0.elapsed_time(e1) * 1e-3
     if world > 1:
         tt = torch.tensor([t_total], device=dev)
@@ -438,7 +441,6 @@ def run_ours(args):
 
     # ---- parity: the result every rank holds after a step, against fp32 torch, on heads picked to cover the launch
     #      order's first and last chunk and (N>1) a head computed by ANOTHER rank and delivered by the exchange ----
-    result = fused.buf if fused is not None else (o_full if world > 1 else out)      # (B,H,S,D) at N>1, local at N=1
     peer_head = None
     if world > 1:
         src = 1                                                  # rank 1's first (batch, head): inputs live there
@@ -631,6 +633,24 @@ def run_ours(args):
         sys.exit(3)
 
 
+DUMP_ROWS = 1 << 16      # sampled rows of O: 32 MiB of float32 at D=128, so out.npy + lse.npy stay under 64 MB
+
+
+def dump_outputs(path, arrays, seed=0):
+    """--dump-outputs: write each array (rows along dim 0) as float32 <path>/<name>.npy.  An array with more than
+    DUMP_ROWS rows is written as the rows at a fixed, seeded sample of DUMP_ROWS indices (ascending), so two builds run
+    with the same arguments can be compared element for element; at N=1, out.npy[i] and lse.npy[i] are the same query
+    row (b, h, s)."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        if t.shape[0] > DUMP_ROWS:
+            idx = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(seed))[:DUMP_ROWS].sort().values
+            t = t[idx.to(t.device)]
+        np.save(os.path.join(path, name + ".npy"), t.float().cpu().numpy())
+
+
 def q_bytes(B, H, S, D):
     return B * H * S * D * 2
 
@@ -744,6 +764,9 @@ def main():
     ap.add_argument("--exchange", default="fused", choices=["fused", "nccl"],
                     help="N>1: how O is gathered (fused peer stores in the kernel epilogue, or ncclAllGather)")
     ap.add_argument("--chunks", type=int, default=1, help="N>1: batch chunks per rank (gather/compute overlap)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's O and LSE at a fixed sample of query rows "
+                         "as DIR/out.npy and DIR/lse.npy (float32)")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference_arm(args)

@@ -18,12 +18,16 @@ import json
 import math
 import os
 import sys
+import tempfile
 import time
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "baseline", "_ref"))
-# flashinfer JIT cache pre-built in the CPU container (baseline/prebuild_flashinfer.py); same absolute path on the box
-os.environ.setdefault("FLASHINFER_WORKSPACE_BASE", "/root/repo/baseline/_ref/flashinfer_ws")
+# flashinfer JIT-compiles its FMHA module on first use; unless the caller names a cache, that build goes to a temporary
+# directory removed at exit, so bench.py writes nothing into the tree (which may be read-only)
+if "FLASHINFER_WORKSPACE_BASE" not in os.environ:
+    _FLASHINFER_WS = tempfile.TemporaryDirectory(prefix="tfa_flashinfer_")
+    os.environ["FLASHINFER_WORKSPACE_BASE"] = _FLASHINFER_WS.name
 
 import torch  # noqa: E402
 

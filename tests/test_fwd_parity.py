@@ -181,7 +181,7 @@ def test_deterministic(tfa):
     assert torch.equal(a, b) and torch.equal(la, lb)
 
 
-def test_classic_and_persistent_kernels_agree_bitwise(tfa):
+def test_classic_and_persistent_kernels_agree_bitwise(tfa, tmp_path):
     """The kernel is selected per process (TFA_KERNEL): the one-CTA-per-item kernel and the persistent kernel do the same
     arithmetic in the same order, so one causal and one ragged case must agree bit for bit (different schedules, TMA-store
     vs st.global epilogue)."""
@@ -203,10 +203,10 @@ for (B, H, S, D, causal) in ((2, 5, 1280, 128, True), (1, 3, 333, 64, False)):
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     outs = {}
     for variant in ("classic", "persist"):
-        env = dict(os.environ, TFA_ROOT=root, TFA_OUT=f"/tmp/tfa_variant_{variant}")
+        env = dict(os.environ, TFA_ROOT=root, TFA_OUT=str(tmp_path / variant))
         env["TFA_KERNEL"] = variant
         p = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=600)
         assert p.returncode == 0, p.stderr[-2000:]
-        outs[variant] = [torch.load(f"/tmp/tfa_variant_{variant}_{S}.pt") for S in (1280, 333)]
+        outs[variant] = [torch.load(tmp_path / f"{variant}_{S}.pt") for S in (1280, 333)]
     for (a, la), (b, lb) in zip(outs["classic"], outs["persist"]):
         assert torch.equal(a, b) and torch.equal(la, lb)
