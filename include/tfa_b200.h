@@ -50,7 +50,7 @@ extern "C" {
 #define TFA_EDEVICE_FAULT (-8)  /* kernel watchdog fired; see tfa_debug_record()  */
 #define TFA_EINVAL_SCALE  (-9)  /* softmax_scale negative, NaN or infinite         */
 #define TFA_EINVAL_HEADS  (-10) /* Hq not a multiple of Hkv                         */
-#define TFA_EINVAL_WORKSPACE (-11) /* split-KV asked for but workspace missing/small */
+#define TFA_EINVAL_WORKSPACE (-11) /* workspace missing, misaligned or too small      */
 
 /* Extended argument block (POD), the analogue of Flash_fwd_params (flash.h:29-60).
  * Strides are in ELEMENTS.  The innermost (head_dim) stride must be 1.
@@ -133,6 +133,39 @@ int tfa_attn_fwd(const tfa_attn_args* args);
 int tfa_attn_num_splits(const tfa_attn_args* args);
 /* Workspace needed for `num_splits` (as returned above): num_splits * B*Hq*Sq * (D + 1) * 4 bytes; 0 for 1. */
 size_t tfa_attn_workspace_bytes(const tfa_attn_args* args, int num_splits);
+
+/* ---- backward of the tfa_fwd_ex problem (MHA, Sq == Sk, D in {64, 128}, top-left causal or none) ----
+ *   P = exp(scale * Q K^T - lse) (masked), Delta_i = sum_d dO_id * O_id,
+ *   dV = P^T dO,  dS = P o (dO V^T - Delta),  dQ = scale * dS K,  dK = scale * dS^T Q.
+ * P and dS are rounded to the input dtype before their matrix products; accumulation is fp32.
+ * q, k, v, out (the forward's O), dout (dO), dq, dk and dv all use the one stride triple (elements, unit head_dim
+ * stride), so (B,H,S,D) and (B,S,H,D) both work.  lse is the forward's (B,H,S) contiguous fp32 output.
+ * Every pointer, lse and workspace included, must be non-NULL and 16-byte aligned.
+ * Two kernels are launched asynchronously on `stream` (dQ and Delta, then dK and dV); the result is bitwise
+ * deterministic.  workspace: device memory of at least tfa_bwd_workspace_bytes() bytes (Delta, fp32),
+ * otherwise TFA_EINVAL_WORKSPACE. */
+typedef struct tfa_bwd_args {
+  const void* q;
+  const void* k;
+  const void* v;
+  const void* out;          /* O of the forward                      */
+  const void* dout;         /* dO                                    */
+  const float* lse;         /* (B,H,S) fp32 of the forward, required */
+  void* dq;
+  void* dk;
+  void* dv;
+  int32_t B, H, S, D;
+  int64_t stride_b, stride_h, stride_s;   /* elements, shared by all eight tensors */
+  int32_t dtype, is_causal;
+  float softmax_scale;
+  void* workspace;
+  size_t workspace_bytes;
+  void* stream;             /* cudaStream_t */
+} tfa_bwd_args;
+
+int tfa_bwd(const tfa_bwd_args* args);
+/* Workspace tfa_bwd() needs: B*H*S*4 bytes (Delta); 0 for a NULL args or an empty shape. */
+size_t tfa_bwd_workspace_bytes(const tfa_bwd_args* args);
 
 /* Host-buffer forward: q/k/v/out/lse are HOST pointers ((B,H,S,D) contiguous; pinned
  * memory gives full PCIe speed).  Copies in, runs tfa_fwd per (batch*head) chunk on

@@ -34,7 +34,8 @@ LIB_NAME = "libtfa_b200.so"
 EXT_NAME = "attention_cutlass" + (sysconfig.get_config_var("EXT_SUFFIX") or ".so")
 
 CU_SOURCES = ["tfa_api.cu", "tfa_selftest.cu", "tfa_microbench.cu"]
-CU_HEADERS = ["ptx_sm100.cuh", "fa_fwd_sm100.cuh", "fa_fwd_sm100_persist.cuh", "fa_splitkv_combine.cuh"]
+CU_HEADERS = ["ptx_sm100.cuh", "fa_fwd_sm100.cuh", "fa_fwd_sm100_persist.cuh", "fa_splitkv_combine.cuh",
+              "fa_bwd_sm100.cuh"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-O3", "-std=c++17", "-lineinfo",

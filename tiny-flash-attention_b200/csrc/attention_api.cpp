@@ -196,6 +196,62 @@ std::vector<torch::Tensor> flash_attention_v2_general(torch::Tensor q, torch::Te
   return {out, lse};
 }
 
+// Backward of flash_attention_v2_cutlass: gradients of q, k, v from dO, the forward's inputs, its output and its
+// softmax_lse.  All (B,H,S,D) contiguous CUDA tensors except softmax_lse, which is (B,H,S) fp32.
+std::vector<torch::Tensor> flash_attention_v2_bwd(torch::Tensor dout, torch::Tensor q, torch::Tensor k,
+                                                  torch::Tensor v, torch::Tensor out, torch::Tensor softmax_lse,
+                                                  bool is_causal, float softmax_scale) {
+  TFA_CHECK_INPUT(dout);
+  TFA_CHECK_INPUT(q);
+  TFA_CHECK_INPUT(k);
+  TFA_CHECK_INPUT(v);
+  TFA_CHECK_INPUT(out);
+  TFA_CHECK_INPUT(softmax_lse);
+  check_common(q, k, v);
+  TORCH_CHECK(out.sizes() == q.sizes() && dout.sizes() == q.sizes(), "out and dout must have the shape of q");
+  TORCH_CHECK(out.scalar_type() == q.scalar_type() && dout.scalar_type() == q.scalar_type(),
+              "out and dout must have the dtype of q");
+  TORCH_CHECK(out.device() == q.device() && dout.device() == q.device() && softmax_lse.device() == q.device(),
+              "dout, q, k, v, out, softmax_lse must be on the same device");
+  const int64_t B = q.size(0), H = q.size(1), S = q.size(2), D = q.size(3);
+  TORCH_CHECK(D == 64 || D == 128, fmt_msg("head_dim must be 64 or 128, got %lld", static_cast<long long>(D)));
+  TORCH_CHECK(B >= 1 && H >= 1 && S >= 1, "empty tensors are not supported");
+  TORCH_CHECK(softmax_lse.scalar_type() == at::kFloat, "softmax_lse must be float32");
+  TORCH_CHECK(softmax_lse.dim() == 3 && softmax_lse.size(0) == B && softmax_lse.size(1) == H && softmax_lse.size(2) == S,
+              fmt_msg("softmax_lse must have shape (%lld, %lld, %lld)", B, H, S));
+
+  torch::Tensor dq, dk, dv, ws;
+  int rc = 0;
+  {
+    // all validation happens above: nothing below throws while the device guard is live
+    c10::cuda::CUDAGuard guard(q.device());
+    dq = torch::empty_like(q);
+    dk = torch::empty_like(k);
+    dv = torch::empty_like(v);
+    tfa_bwd_args a;
+    a.q = q.data_ptr(); a.k = k.data_ptr(); a.v = v.data_ptr();
+    a.out = out.data_ptr(); a.dout = dout.data_ptr(); a.lse = softmax_lse.data_ptr<float>();
+    a.dq = dq.data_ptr(); a.dk = dk.data_ptr(); a.dv = dv.data_ptr();
+    a.B = static_cast<int32_t>(B); a.H = static_cast<int32_t>(H); a.S = static_cast<int32_t>(S);
+    a.D = static_cast<int32_t>(D);
+    a.stride_b = H * S * D; a.stride_h = S * D; a.stride_s = D;
+    a.dtype = q.scalar_type() == at::kBFloat16 ? TFA_BF16 : TFA_FP16;
+    a.is_causal = is_causal ? 1 : 0;
+    a.softmax_scale = softmax_scale;
+    a.workspace = nullptr; a.workspace_bytes = 0;
+    a.stream = at::cuda::getCurrentCUDAStream(q.device().index()).stream();
+    const size_t need = tfa_bwd_workspace_bytes(&a);
+    // freed on return while the kernels may still run: the caching allocator only hands the block out again in
+    // this stream's order
+    ws = torch::empty({static_cast<int64_t>((need + 3) / 4)}, q.options().dtype(at::kFloat));
+    a.workspace = ws.data_ptr();
+    a.workspace_bytes = need;
+    rc = tfa_bwd(&a);
+  }
+  raise_on_error(rc);
+  return {dq, dk, dv};
+}
+
 PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
   m.def("flash_attention_v2_cutlass", &flash_attention_v2_cutlass,
         "Flash attention v2 forward, B200-native (sm_100a tcgen05/TMEM/TMA)");
@@ -205,6 +261,8 @@ PYBIND11_MODULE(TORCH_EXTENSION_NAME, m) {
   m.def("flash_attention_v2_fp32out", &flash_attention_v2_fp32out, "same op, fp32 output (validation)");
   m.def("flash_attention_v2_general", &flash_attention_v2_general,
         "grouped K/V heads, Sq != Sk (bottom-right causal), optional split-KV: (q, k, v, is_causal, scale, num_splits)");
+  m.def("flash_attention_v2_bwd", &flash_attention_v2_bwd,
+        "backward of flash_attention_v2_cutlass: (dout, q, k, v, out, softmax_lse, is_causal, scale) -> [dq, dk, dv]");
   m.def("launch_count", []() { return tfa_launch_count(); }, "kernels launched by the library so far");
   m.def("abi_version", []() { return tfa_abi_version(); });
 }

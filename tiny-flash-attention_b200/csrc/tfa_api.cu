@@ -11,6 +11,7 @@
 #include "fa_fwd_sm100.cuh"
 #include "fa_fwd_sm100_persist.cuh"
 #include "fa_splitkv_combine.cuh"
+#include "fa_bwd_sm100.cuh"
 
 #include <cuda_runtime.h>
 #include <cudaTypedefs.h>
@@ -503,6 +504,89 @@ Problem from_attn_args(const tfa_attn_args& a) {
   return q;
 }
 
+// ---- backward (fa_bwd_sm100.cuh) ----
+int validate_bwd(const tfa_bwd_args& a) {
+  const void* ptrs[9] = {a.q, a.k, a.v, a.out, a.dout, a.lse, a.dq, a.dk, a.dv};
+  for (const void* p : ptrs)
+    if (p == nullptr || (reinterpret_cast<uintptr_t>(p) & 15u)) return TFA_EINVAL_PTR;
+  if (a.D != 64 && a.D != 128) return TFA_EINVAL_DIM;
+  if (a.B < 1 || a.H < 1 || a.S < 1) return TFA_EINVAL_SHAPE;
+  if (a.dtype != TFA_BF16 && a.dtype != TFA_FP16) return TFA_EINVAL_DTYPE;
+  if (!(a.softmax_scale >= 0.0f) || !(a.softmax_scale <= 3.0e38f)) return TFA_EINVAL_SCALE;
+  if (a.stride_s < a.D || (a.stride_s % 8) || (a.stride_h % 8) || (a.stride_b % 8)) return TFA_EINVAL_STRIDE;
+  return 0;
+}
+
+size_t bwd_ws_bytes(const tfa_bwd_args& a) {
+  if (a.B < 1 || a.H < 1 || a.S < 1) return 0;
+  return static_cast<size_t>(a.B) * a.H * a.S * sizeof(float);
+}
+
+template <int D, bool CAUSAL, bool IS_BF16>
+int launch_bwd_inst(const CUtensorMap* tm, const tfa::BwdParams& p, long long nblocks, cudaStream_t stream) {
+  using C = tfa::BwdCfg<D>;
+  cudaError_t cerr;
+  auto kdq = tfa::fa_bwd_dq_kernel<D, CAUSAL, IS_BF16>;
+  auto kkv = tfa::fa_bwd_dkdv_kernel<D, CAUSAL, IS_BF16>;
+  if ((cerr = opt_in_smem(kdq, C::SMEM_BYTES)) != cudaSuccess) return static_cast<int>(cerr);
+  if ((cerr = opt_in_smem(kkv, C::SMEM_BYTES)) != cudaSuccess) return static_cast<int>(cerr);
+  // dQ first: it also writes Delta, which the dK/dV kernel reads (stream order)
+  kdq<<<static_cast<int>(nblocks), C::THREADS, C::SMEM_BYTES, stream>>>(tm[0], tm[1], tm[2], tm[3], p);
+  g_launches.fetch_add(1, std::memory_order_relaxed);
+  if ((cerr = cudaGetLastError()) != cudaSuccess) return static_cast<int>(cerr);
+  kkv<<<static_cast<int>(nblocks), C::THREADS, C::SMEM_BYTES, stream>>>(tm[0], tm[1], tm[2], tm[3], p);
+  g_launches.fetch_add(1, std::memory_order_relaxed);
+  return static_cast<int>(cudaGetLastError());
+}
+
+template <int D>
+int dispatch_bwd(bool causal, bool bf16, const CUtensorMap* tm, const tfa::BwdParams& p, long long nblocks,
+                 cudaStream_t s) {
+  if (causal) return bf16 ? launch_bwd_inst<D, true, true>(tm, p, nblocks, s) : launch_bwd_inst<D, true, false>(tm, p, nblocks, s);
+  return bf16 ? launch_bwd_inst<D, false, true>(tm, p, nblocks, s) : launch_bwd_inst<D, false, false>(tm, p, nblocks, s);
+}
+
+int bwd_impl(const tfa_bwd_args& a) {
+  int rc = validate_bwd(a);
+  if (rc) return rc;
+  const size_t need = bwd_ws_bytes(a);
+  if (a.workspace == nullptr || (reinterpret_cast<uintptr_t>(a.workspace) & 15u) || a.workspace_bytes < need)
+    return TFA_EINVAL_WORKSPACE;
+  const long long ntiles = (static_cast<long long>(a.S) + 127) / 128;
+  const long long nblocks = ntiles * a.B * a.H;      // both kernels: one CTA per (batch*head, 128-row tile)
+  if (nblocks > 0x7fffffffLL) return TFA_EINVAL_SHAPE;
+  if (!arch_ok()) return TFA_EARCH;
+  init_dbg();
+
+  CUtensorMap tm[4];   // q, k, v, dout
+  const void* src[4] = {a.q, a.k, a.v, a.dout};
+  for (int i = 0; i < 4; ++i)
+    if ((rc = make_tmap(&tm[i], src[i], a.dtype, a.D, a.S, a.B, a.H, a.stride_b, a.stride_h, a.stride_s))) return rc;
+
+  tfa::BwdParams p;
+  std::memset(&p, 0, sizeof(p));
+  p.out = a.out;
+  p.dout = a.dout;
+  p.lse = a.lse;
+  p.delta = static_cast<float*>(a.workspace);
+  p.dq = a.dq;
+  p.dk = a.dk;
+  p.dv = a.dv;
+  p.stride_b = a.stride_b;
+  p.stride_h = a.stride_h;
+  p.stride_s = a.stride_s;
+  p.H = a.H;
+  p.S = a.S;
+  p.ntiles = static_cast<int>(ntiles);
+  p.scale = a.softmax_scale;
+  p.scale_log2 = fmaxf(a.softmax_scale * 1.4426950408889634f, 1.0e-30f);   // the forward's clamp (fwd_impl)
+  p.dbg = g_dbg_dev;
+  const bool causal = a.is_causal != 0, bf16 = a.dtype == TFA_BF16;
+  cudaStream_t stream = static_cast<cudaStream_t>(a.stream);
+  return (a.D == 64) ? dispatch_bwd<64>(causal, bf16, tm, p, nblocks, stream)
+                     : dispatch_bwd<128>(causal, bf16, tm, p, nblocks, stream);
+}
+
 // ---- host-buffer path workspace ----
 struct HostWs {
   void* d[4] = {nullptr, nullptr, nullptr, nullptr};   // q k v o
@@ -555,6 +639,16 @@ int tfa_fwd_multi(const tfa_fwd_args* args, void* const* extra_out, int n_extra)
   if (!args) return TFA_EINVAL_PTR;
   if (n_extra < 0) return TFA_EINVAL_SHAPE;
   return fwd_impl(from_fwd_args(*args), extra_out, n_extra);
+}
+
+int tfa_bwd(const tfa_bwd_args* args) {
+  if (!args) return TFA_EINVAL_PTR;
+  return bwd_impl(*args);
+}
+
+size_t tfa_bwd_workspace_bytes(const tfa_bwd_args* args) {
+  if (!args) return 0;
+  return bwd_ws_bytes(*args);
 }
 
 int tfa_fwd(const void* q, const void* k, const void* v, void* out, float* lse, int B, int H, int S, int D, int dtype,
@@ -697,7 +791,8 @@ const char* tfa_error_string(int code) {
     case TFA_EDEVICE_FAULT: return "tfa: kernel watchdog fired (see tfa_debug_record)";
     case TFA_EINVAL_SCALE: return "tfa: softmax_scale must be finite and >= 0";
     case TFA_EINVAL_HEADS: return "tfa: query heads must be a multiple of K/V heads";
-    case TFA_EINVAL_WORKSPACE: return "tfa: split-KV needs a 16-byte aligned workspace of tfa_attn_workspace_bytes()";
+    case TFA_EINVAL_WORKSPACE:
+      return "tfa: workspace missing, not 16-byte aligned or smaller than tfa_attn_workspace_bytes() / tfa_bwd_workspace_bytes()";
     default: return code > 0 ? cudaGetErrorString(static_cast<cudaError_t>(code)) : "tfa: unknown error";
   }
 }

@@ -14,7 +14,7 @@ LIB_PATH = os.environ.get("TFA_LIB", os.path.join(HERE, "libtfa_b200.so"))   # T
 
 TFA_BF16, TFA_FP16 = 0, 1
 _LIB = None
-_WORKSPACES = {}     # (device, stream) -> last split-KV workspace, see attn_fwd()
+_WORKSPACES = {}     # (device, stream) -> last split-KV workspace, see attn_fwd(); (device, stream, "bwd"): bwd()
 
 
 class TfaError(RuntimeError):
@@ -50,6 +50,19 @@ class AttnArgs(ctypes.Structure):
     ]
 
 
+class BwdArgs(ctypes.Structure):
+    """struct tfa_bwd_args (include/tfa_b200.h)."""
+    _fields_ = [
+        ("q", ctypes.c_void_p), ("k", ctypes.c_void_p), ("v", ctypes.c_void_p), ("out", ctypes.c_void_p),
+        ("dout", ctypes.c_void_p), ("lse", ctypes.c_void_p),
+        ("dq", ctypes.c_void_p), ("dk", ctypes.c_void_p), ("dv", ctypes.c_void_p),
+        ("B", ctypes.c_int32), ("H", ctypes.c_int32), ("S", ctypes.c_int32), ("D", ctypes.c_int32),
+        ("stride_b", ctypes.c_int64), ("stride_h", ctypes.c_int64), ("stride_s", ctypes.c_int64),
+        ("dtype", ctypes.c_int32), ("is_causal", ctypes.c_int32), ("softmax_scale", ctypes.c_float),
+        ("workspace", ctypes.c_void_p), ("workspace_bytes", ctypes.c_size_t), ("stream", ctypes.c_void_p),
+    ]
+
+
 def lib():
     global _LIB
     if _LIB is None:
@@ -71,6 +84,10 @@ def lib():
         L.tfa_attn_num_splits.restype = ci
         L.tfa_attn_workspace_bytes.argtypes = [ctypes.POINTER(AttnArgs), ci]
         L.tfa_attn_workspace_bytes.restype = ctypes.c_size_t
+        L.tfa_bwd.argtypes = [ctypes.POINTER(BwdArgs)]
+        L.tfa_bwd.restype = ci
+        L.tfa_bwd_workspace_bytes.argtypes = [ctypes.POINTER(BwdArgs)]
+        L.tfa_bwd_workspace_bytes.restype = ctypes.c_size_t
         L.tfa_fwd_host.argtypes = [vp, vp, vp, vp, vp, ci, ci, ci, ci, ci, ci, cf, ci]
         L.tfa_fwd_host.restype = ci
         L.tfa_host_release.restype = None
@@ -159,6 +176,35 @@ def attn_fwd(q, k, v, is_causal, softmax_scale, num_splits=1, out_fp32=False, st
     if return_splits:
         return out, lse, n
     return out, lse
+
+
+def bwd(dout, q, k, v, out, lse, is_causal, softmax_scale, layout="bhsd", stream=None):
+    """Gradients (dq, dk, dv) through tfa_bwd(): contiguous device tensors in `layout` ("bhsd" or "bshd"), `lse` the
+    forward's (B,H,S) fp32 output."""
+    import torch
+    for t in (dout, q, k, v, out, lse):
+        assert t.is_cuda and t.is_contiguous(), "contiguous device tensors required"
+    if layout == "bhsd":
+        B, H, S, D = q.shape
+        sb, sh, ss = H * S * D, S * D, D
+    elif layout == "bshd":
+        B, S, H, D = q.shape
+        sb, ss, sh = S * H * D, H * D, D
+    else:
+        raise ValueError(layout)
+    dq, dk, dv = torch.empty_like(q), torch.empty_like(k), torch.empty_like(v)
+    st = stream if stream is not None else torch.cuda.current_stream(q.device).cuda_stream
+    a = BwdArgs(q.data_ptr(), k.data_ptr(), v.data_ptr(), out.data_ptr(), dout.data_ptr(), lse.data_ptr(),
+                dq.data_ptr(), dk.data_ptr(), dv.data_ptr(), B, H, S, D, sb, sh, ss, _dtype_code(q),
+                int(bool(is_causal)), float(softmax_scale), None, 0, st)
+    L = lib()
+    need = int(L.tfa_bwd_workspace_bytes(ctypes.byref(a)))
+    ws = torch.empty((need + 3) // 4, dtype=torch.float32, device=q.device)
+    a.workspace, a.workspace_bytes = ws.data_ptr(), need
+    # keep the workspace alive until the next call on the same stream (the launch is asynchronous)
+    _WORKSPACES[(q.device.index, int(st), "bwd")] = ws
+    check(L.tfa_bwd(ctypes.byref(a)))
+    return dq, dk, dv
 
 
 def fwd_multi(q, k, v, is_causal, softmax_scale, out, extra_ptrs, lse=None, stream=None):
